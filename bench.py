@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the APTP hot path: mixed-expert gated SD-2.1 U-Net denoising step on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one U-Net forward over one batch of synthetic input (BASELINE.json configs[1]: bf16,
 batch 64 per GPU, 64x64 latent, 8 architecture codes with width + depth gating, random-init weights).
@@ -148,6 +148,34 @@ def finish_dist():
         dist.destroy_process_group()
 
 
+def dump_outputs(args, world, rank, **arrays):
+    """--dump-outputs DIR: each array as DIR/<name>.npy in float32, or DIR/<name>_rank<k>.npy when several ranks run
+    (every rank draws its own seeded inputs)."""
+    if not args.dump_outputs:
+        return
+    import numpy as np
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(args.dump_outputs, f"{name}{suffix}.npy"), a.detach().float().cpu().numpy())
+
+
+def sampled_entries(tensors, n: int, seed: int = 0):
+    """A fixed, seeded sample of n entries (positions drawn with replacement, sorted) of the concatenation of
+    `tensors`, for outputs too large to store whole."""
+    import torch
+    sizes = torch.tensor([t.numel() for t in tensors])
+    ends = torch.cumsum(sizes, 0)
+    pos = torch.randint(0, int(ends[-1]), (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    which = torch.searchsorted(ends, pos, right=True)
+    off = pos - (ends - sizes)[which]
+    parts = []
+    for i in which.unique().tolist():
+        sel = which == i
+        parts.append(tensors[i].detach().reshape(-1)[off[sel].to(tensors[i].device)].float().cpu())
+    return torch.cat(parts)
+
+
 def make_workload(device, seed):
     import torch
     from diffusion_pruning_b200.synthetic import split_arch, synthetic_codes
@@ -199,11 +227,12 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(ms over `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            y = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -212,7 +241,7 @@ def run_ours(args):
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             ms = float(tt.item())
         barrier()
-        return ms
+        return ms, y
 
     clocks = ClockSampler(local)
     clocks.start()
@@ -225,10 +254,14 @@ def run_ours(args):
         torch.cuda.synchronize()
         torch.cuda.profiler.stop()
     clocks.begin()
-    ms_total = timed(step_resident, args.steps)
+    ms_total, y_last = timed(step_resident, args.steps)
     clocks.end()
     clocks.extend(step_resident)
     clk = clocks.stop()
+    # the forward returns a fresh tensor every step (a graph replay returns a copy of its static output), so y_last
+    # still holds the prediction of the last timed step
+    dump_outputs(args, world, rank, sample=y_last)
+    del y_last
     eng = model._engine
     launches_per_step = eng.launches
     kept_flops = eng.flops
@@ -237,7 +270,7 @@ def run_ours(args):
     for _ in range(2):
         step_e2e()
     t0 = time.perf_counter()
-    ms_e2e_dev = timed(step_e2e, args.steps)
+    ms_e2e_dev, _ = timed(step_e2e, args.steps)
     ms_e2e = ms_e2e_dev
     # per-kernel timing of the dominant kernel, live, with CUDA events on the launching stream
     # (eager launches, each bracketed by two events. The GPU is first parked on a spin kernel so that the host has queued the
@@ -362,7 +395,7 @@ def run_ours(args):
         sec = secondary_workloads(args)
         out["secondary"] = sec
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
-        out["cpu_baseline"] = cpu_baseline(sample_steps=1)
+        out["cpu_baseline"], _ = cpu_baseline(sample_steps=1)
     if rank == 0:
         print(json.dumps(out), flush=True)
 
@@ -462,6 +495,7 @@ def measure_train(args):
         ms = float(tt.item())
     clk = clocks.stop()
     K.check_abort()
+    dump_outputs(args, world, rank, train_loss=loss, train_grad=flat)  # flat: the last step's (reduced) gradients
     peaks = load_peaks()
     value = Bt * world * args.steps / (ms / 1e3)
     tflop_per_sample = 2.52  # SURVEY 8(d): two forwards + dgrad-only backward at 64x64
@@ -565,6 +599,7 @@ def measure_sample(args):
     clk = clocks.stop()
     K.check_abort()
     assert torch.isfinite(result).all(), "sampling produced non-finite latents"
+    dump_outputs(args, world, rank, sample_latents=result, sample_experts=idx)
     value = P * world * STEPS * args.steps / (ms / 1e3)
     if True:
         out = {"metric": "routed_sampling_prompt_steps_per_s", "value": round(value, 2), "unit": "prompts*steps/s",
@@ -668,6 +703,9 @@ def measure_finetune(args):
         ms = float(tt.item())
     clk = clocks.stop()
     K.check_abort()
+    if args.dump_outputs:  # the last step's gradients cover 866 M parameters: a fixed sample of 2^20 of them
+        dump_outputs(args, world, rank, finetune_loss=loss,
+                     finetune_grad_sample=sampled_entries([p.grad for p in params if p.grad is not None], 1 << 20))
     peaks = load_peaks()
     value = Bt * world * args.steps / (ms / 1e3)
     # dense-equivalent FLOPs per sample: teacher forward + student forward + dgrad + wgrad of the conv / linear layers
@@ -767,6 +805,7 @@ def secondary_workloads(args):
     sec = {}
     a = copy.copy(args)
     a.steps, a.warmup = args.secondary_train_steps, 6  # (the allocator re-grows its pools after the library-baseline leg)
+    a.dump_outputs = None  # --dump-outputs records the headline forward only
     try:
         tr = measure_train(a)
         sec.update(train_samples_steps_per_s=tr["value"], train_ms=tr["ms_per_step"], train_batch_per_gpu=a.train_batch,
@@ -777,6 +816,7 @@ def secondary_workloads(args):
     torch.cuda.empty_cache()
     a = copy.copy(args)
     a.steps, a.warmup = 1, 1
+    a.dump_outputs = None
     try:
         sm = measure_sample(a)
         sec.update(sample_prompt_steps_per_s=sm["value"], sample_ms_per_pass=sm["ms_per_step"],
@@ -790,7 +830,8 @@ def secondary_workloads(args):
 
 
 def cpu_baseline(sample_steps: int = 1):
-    """The reference's CPU path (fp32 oracle restatement) on the host cores: config 1 (batch 4, 64x64)."""
+    """The reference's CPU path (fp32 oracle restatement) on the host cores: config 1 (batch 4, 64x64). Returns (numbers,
+    prediction of the last timed forward)."""
     import torch
     from diffusion_pruning_b200.synthetic import split_arch, synthetic_codes
     threads = os.cpu_count() or 1
@@ -810,11 +851,11 @@ def cpu_baseline(sample_steps: int = 1):
         o.set_structure(split_arch(arch.clone(), st))
         t0 = time.perf_counter()
         for _ in range(sample_steps):
-            o(sample, t, ctx)
+            y = o(sample, t, ctx)
         dt = time.perf_counter() - t0
     return {"value": round(4 * sample_steps / dt, 4), "unit": UNIT, "cores": threads, "kind": "port",
             "sample": f"{sample_steps} forward(s) of BASELINE configs[0] (batch 4, 64x64 latent, fp32, hard gates "
-                      f"multiplied as in the reference) on {threads} host threads, {dt:.1f} s"}
+                      f"multiplied as in the reference) on {threads} host threads, {dt:.1f} s"}, y
 
 
 def run_reference(args):
@@ -822,9 +863,10 @@ def run_reference(args):
     if rank != 0:
         return
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    cb = cpu_baseline(sample_steps=max(1, min(args.steps, 3)))
+    cb, y = cpu_baseline(sample_steps=args.steps)
+    dump_outputs(args, 1, rank, reference_sample=y)
     out = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": world,
-           "steps": max(1, min(args.steps, 3)), "warmup": 1, "ms_per_step": round(4e3 / cb["value"], 1),
+           "steps": args.steps, "warmup": 1, "ms_per_step": round(4e3 / cb["value"], 1),
            "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
            "config": {"workload": "configs[1] workload, bounded sample: batch-4 slices (configs[0] size) per step on "
                                   "the host CPU", "latent": LATENT, "codes": N_CODES},
@@ -848,7 +890,14 @@ def main():
     ap.add_argument("--prompts", type=int, default=16, help="--workload sample: prompts per GPU")
     ap.add_argument("--sample-latent", type=int, default=96)
     ap.add_argument("--ddim-steps", type=int, default=25)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as float32 DIR/<name>.npy (DIR/<name>_rank<k>.npy "
+                         "with several ranks): forward sample; train loss + gradients; sample latents + expert per "
+                         "prompt; finetune loss + a fixed sample of the gradients; --impl reference sample. The seeded "
+                         "inputs are the same in every run with the same arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return

@@ -19,7 +19,7 @@ constructor-only stand-ins for their diffusers base classes (oracle/ref_shim/dif
     :641-697, :763-851, :1139-1355, :1427-1438, and the prune sweep of unet_2d_conditional.py:2425-2436;
   * count_ops_and_params + calc_macs (op_counter.py:19-116, :259-306; unet_2d_conditional.py:2124-2163);
 tests/test_oracle_unet_pinned.py holds this file to those outputs bit-for-bit in fp32 (<= 1e-5 where the reference
-slices weights and this file keeps exact-zero gates), and re-runs the reference live when /root/reference exists.
+slices weights and this file keeps exact-zero gates).
 Still restated, hence the only unpinned arithmetic: what the stubs themselves implement -- the container loops the
 reference inherits (resnet -> attention order, skip concatenation, samplers), Transformer2DModel.forward of the
 width-only variant, Downsample2D / Upsample2D, Timesteps / TimestepEmbedding, GEGLU.gelu, and PyTorch 2.11 (not 2.1.0)
