@@ -62,13 +62,10 @@ def check_gemm_linear(M=1000, Kd=320, N=320, bn=160, bias=True, residual=True, s
     _close(out, ref, 2e-2, 1e-2, f"gemm_linear M{M} K{Kd} N{N} bn{bn}")
 
 
-def check_gemm_grouped(seed=0):
-    """3 expert buckets: different kept N / kept K, one depth-dropped; compacted weight blocks."""
-    HW, C, N = 256, 320, 320
-    samples = [3, 2, 4]  # per expert
-    n_valid = [250, 320, 130]
-    k_valid = [192, 320, 70]  # kept input channels (zero-padded to 64 in A and W)
-    active = [True, True, False]
+def check_gemm_grouped(seed=0, HW=256, C=320, N=320, samples=(3, 2, 4), n_valid=(250, 320, 130), k_valid=(192, 320, 70),
+                       active=(True, True, False)):
+    """3 expert buckets: different kept N / kept K, one depth-dropped; compacted weight blocks. With C >= 1280 the
+    launch takes the 2-SM scheme; HW not a multiple of 128 puts bucket starts off the 128-row grid."""
     M = sum(samples) * HW
     a = torch.zeros(M, C, device=DEV, dtype=torch.bfloat16)
     w = torch.zeros(3 * N, C, device=DEV, dtype=torch.bfloat16)
@@ -422,10 +419,11 @@ def check_gemm_res_f32(conv=False, seed=0):
     _close(out, ref, 2e-3, 1e-4, "gemm fp32 out + fp32 residual")
 
 
-def check_gemm_ln_fold(geglu=False, seed=0):
+def check_gemm_ln_fold(geglu=False, seed=0, C=320):
     """LayerNorm folded into the consumer GEMM (APTP_EPI_LN_FOLD) with the row statistics written by the producer GEMM's
-    epilogue (rowstat_out): producer = Linear + residual -> x (bf16); consumer = Linear(LayerNorm(x)) [or GEGLU]."""
-    M, C, N = 1000, 320, 640
+    epilogue (rowstat_out): producer = Linear + residual -> x (bf16); consumer = Linear(LayerNorm(x)) [or GEGLU].
+    C = 1280 runs producer and consumer in the 2-SM scheme."""
+    M, N = 1000, 640
     a0 = _rand(M, C, seed=seed).bfloat16()
     w0 = _rand(C, C, scale=C ** -0.5, seed=seed + 1).bfloat16()
     res = (_rand(M, C, seed=seed + 2) * 2 + 0.7).bfloat16()
@@ -549,6 +547,45 @@ def check_gemm_colstat(conv=False, seed=0):
     assert (stats2[1] == -7.0).all(), "samples with zero channels are skipped"
 
 
+def check_conv_grouped(H=32, W=32, Cin=320, N=320, bn=160, samples=(2, 1, 3), n_valid=(320, 250, 130),
+                       k_valid=(320, 192, 64), active=(True, False, True), seed=0):
+    """3x3 conv over three expert buckets (whole samples each) with different kept Cin / Cout, one depth-dropped, in
+    one launch: 32 x 32 images take the 2-SM halo scheme (8 x 16 boxes), 4 x 4 images 4 x 4 x 8 boxes whose batch
+    extent runs past the bucket (and the batch)."""
+    B = sum(samples)
+    hw = H * W
+    x = torch.zeros(B, H, W, Cin, device=DEV, dtype=torch.bfloat16)
+    wp = torch.zeros(3 * N, 9 * Cin, device=DEV, dtype=torch.bfloat16)
+    bias = torch.zeros(3 * N, device=DEV)
+    out = torch.full((B * hw, N), 7.0, device=DEV, dtype=torch.bfloat16)
+    segs, refs, b0 = [], [], 0
+    for e in range(3):
+        nb, kv, nv = samples[e], k_valid[e], n_valid[e]
+        xe = _rand(nb, kv, H, W, seed=seed + 10 * e).bfloat16()
+        we = _rand(nv, kv, 3, 3, scale=(9 * kv) ** -0.5, seed=seed + 10 * e + 1).bfloat16()
+        be = _rand(nv, seed=seed + 10 * e + 2)
+        x[b0:b0 + nb, :, :, :kv] = xe.permute(0, 2, 3, 1)
+        wp[e * N:e * N + nv].view(nv, 9, Cin)[:, :, :kv] = we.permute(0, 2, 3, 1).reshape(nv, 9, kv)
+        bias[e * N:e * N + nv] = be
+        ns = min((nv + 63) // 64 * 64, N)
+        segs.append(K.Segment(b0 * hw, (b0 + nb) * hw, nv, (kv + 63) // 64, w_row_off=e * N, vec_off=e * N, n_store=ns,
+                              active=active[e]))
+        refs.append((b0 * hw, nb * hw, nv, ns, _conv_ref(xe.float(), we.float(), be, 1)))
+        b0 += nb
+    sched = K.build_schedule(segs, bn, DEV, mode=A_CONV3X3, Ho=H, Wo=W)
+    K.grouped_gemm(x.reshape(B * hw, Cin), wp, out, sched, a_ld=Cin, a_k=Cin, a_rows=B * hw, mode=A_CONV3X3, batch=B,
+                   H=H, W=W, k_tap_pitch=Cin, out_ld=N, bias=bias, rows_per_sample=hw)
+    K.check_abort()
+    for e, (r0, rows, nv, ns, ref) in enumerate(refs):
+        blk = out[r0:r0 + rows].float()
+        if not active[e]:
+            assert (blk == 7.0).all(), f"conv bucket {e}: inactive bucket must not be written"
+            continue
+        _close(blk[:, :nv], ref.permute(0, 2, 3, 1).reshape(rows, nv), 2e-2, 1e-2, f"conv bucket {e} box {sched.box}")
+        assert (blk[:, nv:ns] == 0).all(), f"conv bucket {e}: padding columns must be zero"
+        assert (blk[:, ns:] == 7.0).all(), f"conv bucket {e}: columns past n_store must be untouched"
+
+
 def check_attention(B=2, heads=3, kept=(3, 1), Nq=256, Nkv=256, seed=0):
     C = heads * 64
     q = _rand(B * Nq, C, seed=seed).bfloat16()
@@ -633,6 +670,17 @@ ALL = [
     ("layernorm", lambda: check_layernorm()),
     ("layernorm_1280", lambda: check_layernorm(rows=77, C=1280)),
     ("elementwise", check_elementwise),
+    # 2-SM scheme (taps * K >= 1280) with the features the full-width U-Net combines with it
+    ("geglu_2sm_k1280", lambda: check_geglu(M=600, Kd=1280, inner=1280, n_keep=1000)),
+    ("gemm_ln_fold_2sm", lambda: check_gemm_ln_fold(C=1280)),
+    ("gemm_ln_fold_geglu_2sm", lambda: check_gemm_ln_fold(geglu=True, C=1280)),
+    ("gemm_grouped_2sm_unaligned", lambda: check_gemm_grouped(HW=200, C=1280, N=640, samples=(3, 2, 1),
+                                                               n_valid=(600, 640, 330), k_valid=(1280, 704, 1000),
+                                                               active=(True, False, True))),
+    ("conv3x3_s2_2sm_cin320", lambda: check_conv3x3(B=3, H=32, W=32, Cin=320, Cout=320, bn=160, stride=2, temb=False)),
+    ("conv_grouped_halo", lambda: check_conv_grouped()),
+    ("conv_grouped_4x4x8", lambda: check_conv_grouped(H=4, W=4, Cin=640, N=640, bn=224, samples=(5, 2, 6),
+                                                       n_valid=(640, 600, 320), k_valid=(640, 448, 192))),
     ("attention_self", lambda: check_attention()),
     ("attention_rescale", lambda: check_attention_rescale()),
     ("attention_rescale_ragged", lambda: check_attention_rescale(Nq=384, Nkv=600, seed=5)),
