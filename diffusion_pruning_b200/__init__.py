@@ -2,8 +2,9 @@
 SD-2.1 U-Net denoising step and its router, as hand-written sm_100a CUDA behind the reference's
 `pdm.models` interface. See DESIGN.md / INTEGRATION.md."""
 from .hypernet import HyperStructure
+from .mixture import PrunedExpertMixture
 from .quantizer import StructureVectorQuantizer, hard_concrete
 from .unet import UNet2DConditionModelGated, UNet2DConditionModelPruned, UNet2DConditionOutput
 
 __all__ = ["UNet2DConditionModelGated", "UNet2DConditionModelPruned", "UNet2DConditionOutput", "HyperStructure", "StructureVectorQuantizer",
-           "hard_concrete"]
+           "hard_concrete", "PrunedExpertMixture"]

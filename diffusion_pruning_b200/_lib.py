@@ -17,7 +17,7 @@ c_void_p, c_int, c_int64, c_float = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 class GemmSeg(C.Structure):
     _fields_ = [(n, C.c_int32) for n in
                 ("row_begin", "row_end", "n_valid", "n_store", "k_chunks", "w_row_off", "vec_off", "tab_off",
-                 "out_col_off", "pad0", "pad1", "pad2")]
+                 "out_col_off", "w2_row_off", "pad1", "pad2")]
 
 
 class GemmTile(C.Structure):

@@ -420,7 +420,10 @@ grouped_gemm_kernel(const __grid_constant__ GemmParams p) {
               }
             }
             // the 1x1 shortcut's K steps: plain box of the second tensor into the next A slot, W2 rows = output columns
-            const int b2_row = tile.n0 + (int)cta_rank * (tile_mma_n(seg, tile.n0, p.bn, kGeglu, tile.flags) >> 1);
+            // of this bucket's block in w2 (per-expert shortcut weights). GEGLU launches never carry a2 (the launcher
+            // refuses it); not reading the offset there keeps that instantiation at the parent's 0 spill bytes.
+            const int b2_row = (kGeglu ? 0 : seg.w2_row_off) + tile.n0 +
+                               (int)cta_rank * (tile_mma_n(seg, tile.n0, p.bn, kGeglu, tile.flags) >> 1);
             for (int kc = 0; kc < p.k2_chunks && ok; ++kc) {
               if (!mbar_wait(&aempty_bar[aslot], aphase ^ 1, p.abort_flag) ||
                   !mbar_wait(&empty_bar[stage], phase ^ 1, p.abort_flag)) {

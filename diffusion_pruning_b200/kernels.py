@@ -71,6 +71,7 @@ class Segment:
     n_store: int = -1  # default: n_valid rounded up to 8
     out_col_off: int = 0
     active: bool = True
+    w2_row_off: int = 0  # first row of the bucket's block in the second operand pair's weights (fused shortcut)
 
 
 @dataclass
@@ -173,8 +174,8 @@ def build_schedule(segments: Sequence[Segment], bn: int, device, mode: int = A_L
     out_elems = 0.0
     for si, s in enumerate(segments):
         n_store = s.n_store if s.n_store >= 0 else (s.n_valid + 7) // 8 * 8
-        segs[si, :9] = (s.row_begin, s.row_end, s.n_valid, n_store, s.k_chunks, s.w_row_off, s.vec_off, s.tab_off,
-                        s.out_col_off)
+        segs[si, :10] = (s.row_begin, s.row_end, s.n_valid, n_store, s.k_chunks, s.w_row_off, s.vec_off, s.tab_off,
+                         s.out_col_off, s.w2_row_off)
         if not s.active or s.row_end <= s.row_begin or s.n_valid <= 0 or s.k_chunks <= 0:
             continue
         n_tiles_n = (max(s.n_valid, n_store) + cols_per_tile - 1) // cols_per_tile

@@ -99,6 +99,9 @@ class ExpertSet:
     sample_expert: np.ndarray    # [Bg] expert id of each gate row
     width_starts: List[int]      # arch column of each width gate (len n_gates + 1)
     n_width: int
+    # [E] weight source of each expert (PrunedExpertMixture: the fine-tuned model it runs on; two experts may share a
+    # code and still differ here). None: one source for every expert, the model being run.
+    source: Optional[np.ndarray] = None
 
     @property
     def n_experts(self) -> int:
@@ -111,8 +114,11 @@ class ExpertSet:
     def depth_bits(self, depth_idx: int) -> np.ndarray:
         return self.codes[:, self.n_width + depth_idx]
 
+    def sources(self) -> np.ndarray:
+        return self.source if self.source is not None else np.zeros(self.n_experts, dtype=np.int64)
+
     def key(self) -> bytes:
-        return self.codes.tobytes()
+        return self.codes.tobytes() + (b"" if self.source is None else self.source.astype(np.int64).tobytes())
 
 
 @dataclass
@@ -138,13 +144,14 @@ class BatchLayout:
         return BatchLayout(perm=perm, inv_perm=inv, expert_of_pos=eid[perm], starts=starts, batch=batch)
 
 
-def kept_variants(bits: np.ndarray) -> Tuple[List[np.ndarray], np.ndarray]:
-    """bits [E, w] 0/1 -> (list of distinct kept-index arrays, variant id per expert)."""
-    variants: Dict[bytes, int] = {}
+def kept_variants(bits: np.ndarray, source: Optional[np.ndarray] = None) -> Tuple[List[np.ndarray], np.ndarray]:
+    """bits [E, w] 0/1 -> (list of distinct kept-index arrays, variant id per expert). With `source` [E], experts of
+    different weight sources never share a variant (their compacted blocks hold different weights)."""
+    variants: Dict[tuple, int] = {}
     kept: List[np.ndarray] = []
     vid = np.zeros(bits.shape[0], dtype=np.int64)
     for e in range(bits.shape[0]):
-        k = bits[e].tobytes()
+        k = (int(source[e]) if source is not None else 0, bits[e].tobytes())
         if k not in variants:
             variants[k] = len(kept)
             kept.append(np.nonzero(bits[e])[0])

@@ -41,16 +41,25 @@ def route_prompts(hyper_net, quantizer, prompt_embeddings: torch.Tensor) -> Tupl
 @torch.no_grad()
 def denoise(unet, hyper_net, arch_vectors: torch.Tensor, latents: torch.Tensor, cond: torch.Tensor,
             uncond: torch.Tensor, num_inference_steps: int = 25, guidance_scale: float = 7.5,
-            acp: Optional[torch.Tensor] = None, prediction_type: str = "v_prediction") -> torch.Tensor:
+            acp: Optional[torch.Tensor] = None, prediction_type: str = "v_prediction", experts=None,
+            expert_index: Optional[torch.Tensor] = None) -> torch.Tensor:
     """The scheduler loop (pruning_pipelines.py:757-820) for one batch of prompts whose hard architecture
-    vectors are `arch_vectors` (any mix of experts). latents [B,4,H,W] fp32 ~ N(0,1) (init_noise_sigma = 1)."""
+    vectors are `arch_vectors` (any mix of experts). latents [B,4,H,W] fp32 ~ N(0,1) (init_noise_sigma = 1).
+    With `experts` (a PrunedExpertMixture) each prompt runs on its fine-tuned expert `expert_index` [B] instead: `unet`,
+    `hyper_net` and `arch_vectors` are not used."""
     B = latents.shape[0]
     if B == 0:
         return latents
     acp = (alphas_cumprod() if acp is None else acp).cpu()
     ts = ddim_timesteps(num_inference_steps)
     ratio = 1000 // num_inference_steps
-    unet.set_structure(hyper_net.transform_structure_vector(arch_vectors))   # gates tile over [uncond; cond]
+    if experts is None:
+        unet.set_structure(hyper_net.transform_structure_vector(arch_vectors))   # gates tile over [uncond; cond]
+        model = unet
+    else:
+        if expert_index is None or expert_index.shape != (B,):
+            raise ValueError(f"experts= needs expert_index [{B}] (one expert per prompt)")
+        model = lambda x, t, e: experts(x, t, e, expert_index)  # noqa: E731  (the index tiles over [uncond; cond])
     emb = torch.cat([uncond, cond], dim=0)                                   # :764-765
     x = latents.float().contiguous()
     x2 = torch.empty(2 * B, *x.shape[1:], device=x.device, dtype=torch.float32)
@@ -59,7 +68,7 @@ def denoise(unet, hyper_net, arch_vectors: torch.Tensor, latents: torch.Tensor, 
         x2[:B].copy_(x)                                                      # :792 cat([latents] * 2)
         x2[B:].copy_(x)
         tt = torch.full((2 * B,), float(t), device=x.device)
-        pred = unet(x2, tt, emb).sample                                      # :796-802
+        pred = model(x2, tt, emb).sample                                     # :796-802
         prev = t - ratio
         a_t = float(acp[t])
         a_prev = float(acp[prev]) if prev >= 0 else float(acp[0])            # set_alpha_to_one = False
@@ -111,14 +120,26 @@ def _all_to_all_rows(t: torch.Tensor, send_counts: List[int], recv_counts: List[
 @torch.no_grad()
 def routed_sampling(unet, hyper_net, quantizer, prompt_embeddings: torch.Tensor, latents: torch.Tensor,
                     cond: torch.Tensor, uncond: torch.Tensor, num_inference_steps: int = 25,
-                    guidance_scale: float = 7.5, acp: Optional[torch.Tensor] = None, dispatch: str = "balanced"):
+                    guidance_scale: float = 7.5, acp: Optional[torch.Tensor] = None, dispatch: str = "balanced",
+                    experts=None, code_to_expert: Optional[torch.Tensor] = None):
     """BASELINE configs[3]: route local prompts, dispatch them (all-to-all over NVLink) to the GPU chosen by
     plan_dispatch -- the rank(s) serving their expert, load-balanced --, denoise there, return the final latents to
-    the rank that asked. Returns (latents, code index)."""
+    the rank that asked. Returns (latents, code index).
+    With `experts` (a PrunedExpertMixture, held whole by every rank) each prompt is denoised by the fine-tuned expert of
+    its routed code: `code_to_expert` [n_codes] maps a code index to a mixture position (default:
+    experts.code_to_expert(quantizer.n_e), from the experts' code ids). Routing and dispatch are unchanged."""
     arch, idx = route_prompts(hyper_net, quantizer, prompt_embeddings)
+    eidx = None
+    if experts is not None:
+        cmap = experts.code_to_expert(quantizer.n_e) if code_to_expert is None else torch.as_tensor(code_to_expert)
+        eidx = cmap.to(idx.device, torch.int64)[idx]
+        if bool((eidx < 0).any()):
+            raise ValueError(f"prompts were routed to codes without a fine-tuned expert: "
+                             f"{sorted(set(idx[eidx < 0].tolist()))}")
     world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     if world == 1:
-        return denoise(unet, hyper_net, arch, latents, cond, uncond, num_inference_steps, guidance_scale, acp), idx
+        kw = {} if experts is None else dict(experts=experts, expert_index=eidx)
+        return denoise(unet, hyper_net, arch, latents, cond, uncond, num_inference_steps, guidance_scale, acp, **kw), idx
     owner = plan_dispatch(idx, quantizer.n_e, dispatch)
     order = torch.argsort(owner, stable=True)
     send = torch.bincount(owner, minlength=world)
@@ -126,8 +147,11 @@ def routed_sampling(unet, hyper_net, quantizer, prompt_embeddings: torch.Tensor,
     dist.all_to_all_single(recv, send)
     sc, rc = send.tolist(), recv.tolist()
     payload = [arch[order], latents[order].float(), cond[order], uncond[order]]
-    arch_r, lat_r, cond_r, unc_r = [_all_to_all_rows(p, sc, rc) for p in payload]
-    out_r = denoise(unet, hyper_net, arch_r, lat_r, cond_r, unc_r, num_inference_steps, guidance_scale, acp)
+    if eidx is not None:
+        payload.append(eidx[order])
+    arch_r, lat_r, cond_r, unc_r, *eidx_r = [_all_to_all_rows(p, sc, rc) for p in payload]
+    kw = {} if experts is None else dict(experts=experts, expert_index=eidx_r[0])
+    out_r = denoise(unet, hyper_net, arch_r, lat_r, cond_r, unc_r, num_inference_steps, guidance_scale, acp, **kw)
     back = _all_to_all_rows(out_r, rc, sc)
     out = torch.empty_like(back)
     out[order] = back

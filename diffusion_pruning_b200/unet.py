@@ -794,8 +794,15 @@ class UNet2DConditionModelPruned(UNet2DConditionModelGated):
 
 
 class _Engine:
-    def __init__(self, model: UNet2DConditionModelGated, device):
+    def __init__(self, model: UNet2DConditionModelGated, device, sources: Optional[Sequence[nn.Module]] = None,
+                 gates: Optional[Any] = None):
+        """`model` gives the module tree and config. `sources`: models of that same tree whose parameters the packs are
+        built from, one per weight source (a bucket's source is ExpertSet.source; default: the model alone). `gates`:
+        the owner of the gate state (`_gate_state` / `_flat_gates`; default: the model)."""
         self.m = model
+        self.srcs = list(sources) if sources is not None else [model]
+        self.gates = gates if gates is not None else model
+        self.src_of = np.zeros(1, dtype=np.int64)  # weight source of each expert bucket of the current forward
         self.device = device
         self.dense: Dict[str, Dict[str, torch.Tensor]] = {}
         self.expert: Dict[Tuple[bytes, str], Dict[str, Any]] = {}
@@ -903,7 +910,7 @@ class _Engine:
 
     def _prepare_gates(self, B: int):
         m = self.m
-        st = m._gate_state
+        st = self.gates._gate_state
         if st is None:
             flat_w, flat_d = m._flat_gates
             bg = flat_w[0].shape[0]
@@ -919,11 +926,12 @@ class _Engine:
                 uniq, inv = np.unique(codes, axis=0, return_inverse=True)
                 st["eset"] = P.ExpertSet(codes=uniq, sample_expert=inv.reshape(-1), width_starts=st["width_starts"],
                                          n_width=st["n_width"])
-            m._gate_state = st
+            self.gates._gate_state = st
         assert B % st["bg"] == 0, f"batch {B} is not a multiple of the gate batch {st['bg']}"
         self.compact = st["hard"]
         if self.compact:
             self.eset = st["eset"]
+            self.src_of = self.eset.sources()
             # Cached state (schedules, per-position tables, CUDA graph) is keyed on the BUCKET SIZES of the batch, not
             # on which sample went to which expert: a new prompt -> expert assignment with the same sizes only rewrites
             # the two permutation index buffers (device-resident, read by the gathers at the entry / exit of the forward,
@@ -949,7 +957,9 @@ class _Engine:
             if self.eset.key() in self._esets:
                 self._esets.move_to_end(self.eset.key())
         else:
+            assert len(self.srcs) == 1, "several weight sources need hard (0/1) codes"
             self.eset, self.layout = None, None
+            self.src_of = np.zeros(1, dtype=np.int64)
             self._sid = self._lru_id(self._states, (B, b"soft"), self.MAX_STATES, "st", self.sched)
             self._eid = self._lru_id(self._esets, b"soft", self.MAX_ESETS, "es", self.expert)
             arch = st["arch"]
@@ -1006,15 +1016,64 @@ class _Engine:
             return np.ones(self.eset.n_experts if self.compact else 1, dtype=bool)
         return self.eset.depth_bits(d).astype(bool)
 
+    # ---- weight sources ------------------------------------------------------------------------------
+    def _src_mod(self, mod: nn.Module, s: int) -> nn.Module:
+        """The module of weight source `s` at the place `mod` (a module of self.m) has in the tree."""
+        src = self.srcs[s]
+        if src is self.m:
+            return mod
+        names = self.__dict__.get("_mod_names")
+        if names is None:
+            names = self._mod_names = {id(v): k for k, v in self.m.named_modules()}
+        return src.get_submodule(names[id(mod)])
+
+    def _src_stack(self, mod: nn.Module, fn) -> torch.Tensor:
+        """fn(module of source s) for every source, concatenated along dim 0 in source order (block s of a stacked
+        per-source tensor; a bucket finds its block at src_of * block size)."""
+        parts = [fn(self._src_mod(mod, s)) for s in range(len(self.srcs))]
+        return parts[0] if len(parts) == 1 else torch.cat(parts, 0).contiguous()
+
+    def _src_off(self, block: int) -> np.ndarray:
+        """[E] offset of each bucket's block in a per-source stacked tensor of `block` rows / floats per source."""
+        return self.src_of * int(block)
+
+    def _src_seg(self):
+        """Per-sample affine row (weight source) for GroupNorms whose affine is stacked per source; None with one."""
+        if len(self.srcs) == 1:
+            return None
+        return self._sched(("src_seg",), lambda: self._per_pos(self.src_of))
+
+    def _variant_packs(self, vid: np.ndarray, kept: List[np.ndarray], build) -> Dict[str, torch.Tensor]:
+        """Per-variant weight blocks, each built from the weights of its variant's own source. build(s, kept lists of
+        the variants of source s) returns a dict of tensors holding one equal-sized block per variant along dim 0;
+        the result holds the blocks of every variant in variant order."""
+        vsrc = np.asarray([self.src_of[np.nonzero(vid == v)[0][0]] for v in range(len(kept))])
+        srcs = np.unique(vsrc)
+        if len(srcs) == 1:
+            return build(int(srcs[0]), kept)
+        parts = []
+        for s in srcs:
+            vs = np.nonzero(vsrc == s)[0]
+            parts.append((vs, build(int(s), [kept[v] for v in vs])))
+        out = {}
+        for key in parts[0][1]:
+            blocks: List[Optional[torch.Tensor]] = [None] * len(kept)
+            for vs, d in parts:
+                n = d[key].shape[0] // len(vs)
+                for j, v in enumerate(vs):
+                    blocks[v] = d[key][j * n:(j + 1) * n]
+            out[key] = torch.cat(blocks, 0).contiguous()
+        return out
+
     def _segments(self, hw: int, n_valid, k_chunks, w_row_off, vec_off=None, tab_off=None, n_store=None,
-                  active=None, out_col_off=0) -> List[K.Segment]:
+                  active=None, out_col_off=0, w2_row_off=None) -> List[K.Segment]:
         """One segment per expert bucket (adjacent identical buckets merged)."""
         if not self.compact:
             return [K.Segment(row_begin=0, row_end=self.B * hw, n_valid=int(n_valid[0]), k_chunks=int(k_chunks[0]),
                               w_row_off=int(w_row_off[0]), vec_off=int(vec_off[0]) if vec_off is not None else 0,
                               tab_off=int(tab_off[0]) if tab_off is not None else 0,
                               n_store=int(n_store[0]) if n_store is not None else -1, active=True,
-                              out_col_off=out_col_off)]
+                              out_col_off=out_col_off, w2_row_off=int(w2_row_off[0]) if w2_row_off is not None else 0)]
         segs: List[K.Segment] = []
         st = self.layout.starts
         for e in range(self.eset.n_experts):
@@ -1025,11 +1084,12 @@ class _Engine:
                           vec_off=int(vec_off[e]) if vec_off is not None else 0,
                           tab_off=int(tab_off[e]) if tab_off is not None else 0,
                           n_store=int(n_store[e]) if n_store is not None else -1,
-                          active=bool(active[e]) if active is not None else True, out_col_off=out_col_off)
+                          active=bool(active[e]) if active is not None else True, out_col_off=out_col_off,
+                          w2_row_off=int(w2_row_off[e]) if w2_row_off is not None else 0)
             if segs and segs[-1].row_end == s.row_begin and \
                     (segs[-1].n_valid, segs[-1].k_chunks, segs[-1].w_row_off, segs[-1].vec_off, segs[-1].tab_off,
-                     segs[-1].n_store, segs[-1].active) == (s.n_valid, s.k_chunks, s.w_row_off, s.vec_off, s.tab_off,
-                                                           s.n_store, s.active):
+                     segs[-1].n_store, segs[-1].active, segs[-1].w2_row_off) == \
+                    (s.n_valid, s.k_chunks, s.w_row_off, s.vec_off, s.tab_off, s.n_store, s.active, s.w2_row_off):
                 segs[-1].row_end = s.row_end
             else:
                 segs.append(s)
@@ -1075,16 +1135,27 @@ class _Engine:
 
     # ---- dense (unpruned) weights ---------------------------------------------------------------
     def _dense_linear(self, name: str, lin: nn.Module, n_pad_to: int = 0) -> Dict[str, torch.Tensor]:
-        def build():
-            w = lin.weight.detach()
+        """Unpruned weight + bias, stacked per weight source: a bucket's rows start at src_of * max(n_out, n_pad_to),
+        its bias at src_of * n_out (_dense_offs)."""
+        def weight(l):
+            w = l.weight.detach()
             if w.ndim == 4:
                 w = P.pack_conv_weight(w) if w.shape[-1] == 3 else w.reshape(w.shape[0], w.shape[1])
             w = w.to(self.device, BF16).contiguous()
             if n_pad_to and w.shape[0] < n_pad_to:
                 w = torch.cat([w, torch.zeros(n_pad_to - w.shape[0], w.shape[1], device=self.device, dtype=BF16)], 0)
-            b = lin.bias.detach().to(self.device, torch.float32).contiguous() if lin.bias is not None else None
-            return {"w": w, "b": b}
+            return w
+
+        def build():
+            b = self._src_stack(lin, lambda l: l.bias.detach().to(self.device, torch.float32).contiguous()) \
+                if lin.bias is not None else None
+            return {"w": self._src_stack(lin, weight), "b": b}
         return self._pack(self.dense, name, build)
+
+    def _dense_offs(self, lin: nn.Module, n_pad_to: int = 0) -> Dict[str, np.ndarray]:
+        """Segment offsets of each bucket into a _dense_linear pack of `lin`."""
+        n = lin.weight.shape[0]
+        return dict(w_row_off=self._src_off(max(n, n_pad_to)), vec_off=self._src_off(n))
 
     def linear(self, name: str, lin: nn.Module, x: torch.Tensor, rows: int, k: int, ld: int, out: torch.Tensor,
                out_ld: int, hw: int, *, residual=None, res_ld=0, flags=0, active=None, out_mode=OUT_BF16,
@@ -1096,7 +1167,8 @@ class _Engine:
 
         def build():
             bn = P.choose_bn([n], k=k)
-            segs = self._segments(hw, [n] * E, [(k + 63) // 64] * E, [0] * E, active=active, out_col_off=out_col_off)
+            segs = self._segments(hw, [n] * E, [(k + 63) // 64] * E, active=active, out_col_off=out_col_off,
+                                  **self._dense_offs(lin))
             return K.build_schedule(segs, bn, self.device)
         sched = self._sched(("lin", name, rows, hw), build)
         self._gemm(sched, x, d["w"], out, a_ld=ld, a_k=k, a_rows=rows, out_ld=out_ld, out_mode=out_mode, bias=d["b"],
@@ -1113,7 +1185,7 @@ class _Engine:
 
         def build():
             bn = P.choose_bn([max(cout, 32)], k=9 * cin)
-            segs = self._segments(Ho * Wo, [cout] * E, [(cin + 63) // 64] * E, [0] * E)
+            segs = self._segments(Ho * Wo, [cout] * E, [(cin + 63) // 64] * E, **self._dense_offs(conv, n_pad_to))
             return K.build_schedule(segs, bn, self.device, mode=mode, Ho=Ho, Wo=Wo)
         sched = self._sched(("conv", name, x.B, x.H, x.W), build)
         self._gemm(sched, x.t, d["w"], out, a_ld=x.ld, a_k=x.C, a_rows=x.rows, mode=mode, batch=x.B, H=x.H, W=x.W,
@@ -1198,14 +1270,15 @@ class _Engine:
         tdim = m.time_embedding.linear_2.weight.shape[0]
         w = torch.zeros(E * ntot, tdim, device=self.device, dtype=BF16)
         b = torch.zeros(E * ntot, device=self.device, dtype=torch.float32)
-        for r in m._resnets:
-            off = m._temb_off[r.uid]
-            wt = r.time_emb_proj.weight.detach().to(self.device)
-            bt = (r.time_emb_proj.bias.detach() + r.conv1.bias.detach()).to(self.device, torch.float32)
-            gs = r.cout // r.groups
+        for r0 in m._resnets:
+            off = m._temb_off[r0.uid]
+            gs = r0.cout // r0.groups
             for e in range(E):
+                r = self._src_mod(r0, int(self.src_of[e]))
+                wt = r.time_emb_proj.weight.detach().to(self.device)
+                bt = (r.time_emb_proj.bias.detach() + r.conv1.bias.detach()).to(self.device, torch.float32)
                 if self.compact:
-                    kept = np.nonzero(self.eset.width_bits(self.gate_cols[r.uid]["w"][0])[e])[0]
+                    kept = np.nonzero(self.eset.width_bits(self.gate_cols[r0.uid]["w"][0])[e])[0]
                     rows = torch.as_tensor(P.expand_groups(kept, gs), device=self.device, dtype=torch.long)
                 else:
                     rows = torch.arange(r.cout, device=self.device)
@@ -1234,7 +1307,8 @@ class _Engine:
                                        ("te2", m.time_embedding.linear_2, h, tdim, te)):
             d = self._dense_linear(name, lin)
             sched = self._sched(("te", name), lambda: K.build_schedule(
-                [K.Segment(0, B, tdim, (k + 63) // 64)], P.choose_bn([tdim]), self.device))
+                self._segments(1, [tdim] * E, [(k + 63) // 64] * E, **self._dense_offs(lin)), P.choose_bn([tdim]),
+                self.device))
             self._gemm(sched, src, d["w"], dst, a_ld=k, a_k=k, a_rows=B, out_ld=tdim, bias=d["b"], flags=EPI_SILU,
                        rows_per_sample=1)
         pack = self._temb_pack()
@@ -1290,37 +1364,45 @@ class _Engine:
                     "gamma2": f32(r.norm2.weight).reshape(1, r.cout), "beta2": beta2,
                     "tab": None, "b2": f32(r.conv2.bias), "g1": f32(r.norm1.weight), "b1": f32(r.norm1.bias)}
         gs = r.cout // r.groups
-        w1 = P.pack_conv_weight(r.conv1.weight.detach().to(self.device))
-        w2 = P.pack_conv_weight(r.conv2.weight.detach().to(self.device))
-        g2 = r.norm2.weight.detach().to(self.device, torch.float32)
-        b2 = r.norm2.bias.detach().to(self.device, torch.float32)
         if self.compact:
             bits = self.eset.width_bits(self.gate_cols[r.uid]["w"][0])
-            kept_g, vid = P.kept_variants(bits)
+            kept_g, vid = P.kept_variants(bits, self.eset.source)
         else:
             kept_g, vid = [np.arange(r.groups)], np.zeros(1, dtype=np.int64)
         kept_c = [P.expand_groups(k, gs) for k in kept_g]
-        pruned_c = [np.setdiff1d(np.arange(r.cout), k) for k in kept_c]
         V = len(kept_c)
         d = {"vid": vid, "n1": np.asarray([len(k) for k in kept_c]), "V": V}
-        d["w1"] = P.pack_rows(w1, kept_c, r.cout)
-        d["w2"] = P.pack_cols(w2.to(BF16), kept_c, 9)
-        gam = torch.zeros(V, r.cout, device=self.device)
-        bet = torch.zeros(V, r.cout, device=self.device)
-        for v, k in enumerate(kept_c):
-            idx = torch.as_tensor(k, device=self.device, dtype=torch.long)
-            gam[v, :len(k)] = g2.index_select(0, idx)
-            bet[v, :len(k)] = b2.index_select(0, idx)
-        d["gamma2"], d["beta2"] = gam.contiguous(), bet.contiguous()
-        if self.m.pruned_semantics or not self.compact:
+        with_tab = self.compact and not self.m.pruned_semantics
+
+        def build(s, kept):
+            rs = self._src_mod(r, s)
+            w1 = P.pack_conv_weight(rs.conv1.weight.detach().to(self.device))
+            w2 = P.pack_conv_weight(rs.conv2.weight.detach().to(self.device))
+            g2 = rs.norm2.weight.detach().to(self.device, torch.float32)
+            b2 = rs.norm2.bias.detach().to(self.device, torch.float32)
+            o = {"w1": P.pack_rows(w1, kept, r.cout), "w2": P.pack_cols(w2.to(BF16), kept, 9)}
+            gam = torch.zeros(len(kept), r.cout, device=self.device)
+            bet = torch.zeros(len(kept), r.cout, device=self.device)
+            for v, k in enumerate(kept):
+                idx = torch.as_tensor(k, device=self.device, dtype=torch.long)
+                gam[v, :len(k)] = g2.index_select(0, idx)
+                bet[v, :len(k)] = b2.index_select(0, idx)
+            o["gamma2"], o["beta2"] = gam.contiguous(), bet.contiguous()
+            if with_tab:
+                o["tab"] = P.border_table(rs.conv2.weight.detach().to(self.device), b2,
+                                          [np.setdiff1d(np.arange(r.cout), k) for k in kept])
+            return o
+        d.update(self._variant_packs(vid, kept_c, build))
+        if with_tab:
+            tab = d["tab"]
+            d["tab"] = tab.contiguous() if bool((tab != 0).any().item()) else None
+        else:
             # prune() removed the gated-off channels: nothing of them reaches conv2; soft gates keep every channel
             d["tab"] = None
-        else:
-            tab = P.border_table(r.conv2.weight.detach().to(self.device), b2, pruned_c)
-            d["tab"] = tab.contiguous() if bool((tab != 0).any().item()) else None
-        d["b2"] = r.conv2.bias.detach().to(self.device, torch.float32).contiguous()
-        d["g1"] = r.norm1.weight.detach().to(self.device, torch.float32).contiguous()
-        d["b1"] = r.norm1.bias.detach().to(self.device, torch.float32).contiguous()
+        f32 = lambda p: p.detach().to(self.device, torch.float32).contiguous()  # noqa: E731
+        d["b2"] = self._src_stack(r, lambda rs: f32(rs.conv2.bias))
+        d["g1"] = self._src_stack(r, lambda rs: f32(rs.norm1.weight))
+        d["b1"] = self._src_stack(r, lambda rs: f32(rs.norm1.bias))
         return d
 
     def resnet(self, r: ResnetBlock2DWidthGated, x: Act, skip: Optional[Act] = None) -> Act:
@@ -1361,11 +1443,12 @@ class _Engine:
         xin16 = self.buf("cat", M, r.cin) if r.conv_shortcut is not None else None
         if skip is not None:
             self.groupnorm(x.f, x.C, x.C, B, hw, r.groups, gs_in, r.eps, pk["g1"], pk["b1"], r.cin, a1, r.cin, True,
-                           sample_channels=aux.get("ch_in"), x1=skip.f, c1=skip.C, ld1=skip.C, alg_elems=el_in,
-                           cs0=x.cs, cs1=skip.cs, raw_out=xin16)
+                           sample_seg=self._src_seg(), sample_channels=aux.get("ch_in"), x1=skip.f, c1=skip.C,
+                           ld1=skip.C, alg_elems=el_in, cs0=x.cs, cs1=skip.cs, raw_out=xin16)
         else:
             self.groupnorm(x.f, x.C, x.C, B, hw, r.groups, gs_in, r.eps, pk["g1"], pk["b1"], r.cin, a1, r.cin, True,
-                           sample_channels=aux.get("ch_in"), alg_elems=el_in, cs0=x.cs, raw_out=xin16)
+                           sample_seg=self._src_seg(), sample_channels=aux.get("ch_in"), alg_elems=el_in, cs0=x.cs,
+                           raw_out=xin16)
         # conv1 (N-compacted) + time embedding (+ conv1/time biases, folded into the row vector)
         h1 = self.buf("res_h1", M, r.cout)
 
@@ -1421,8 +1504,10 @@ class _Engine:
         def build_c2():
             bn = P.choose_bn([r.cout], k=9 * int(max(pk["n1"])))
             tab_off = vid * 9 * r.cout
+            # conv2 bias and the fused shortcut's weight rows / bias are stacked per weight source
             segs = self._segments(hw, [r.cout] * E, [(int(n) + 63) // 64 for n in n1_e], vid * r.cout,
-                                  tab_off=tab_off, active=active)
+                                  vec_off=self._src_off(r.cout), tab_off=tab_off, active=active,
+                                  w2_row_off=self._src_off(r.cout))
             return K.build_schedule(segs, bn, self.device, mode=A_CONV3X3, Ho=H, Wo=W)
         sched = self._sched(("res_c2", r.uid, H, W), build_c2)
         cs_out = self._colstat_new(B, H, W, r.cout)
@@ -1468,22 +1553,29 @@ class _Engine:
         C = attn.dim
         is_cross = attn.ctx_dim is not None
         if self.compact:
-            kept_h, vid = P.kept_variants(self.eset.width_bits(gate_idx))
+            kept_h, vid = P.kept_variants(self.eset.width_bits(gate_idx), self.eset.source)
         else:
             kept_h, vid = [np.arange(attn.heads)], np.zeros(1, dtype=np.int64)
         kept_c = [P.expand_groups(k, 64) for k in kept_h]
         d = {"vid": vid, "nh": np.asarray([len(k) for k in kept_h]), "V": len(kept_h)}
-        gam = ln.weight.detach().to(self.device, torch.float32)
-        bet = ln.bias.detach().to(self.device, torch.float32)
-        if not self.ln_fold:
-            gam, bet = torch.ones_like(gam), torch.zeros_like(bet)
-        for nm, lin in (("q", attn.to_q), ("k", attn.to_k), ("v", attn.to_v)):
-            w = lin.weight.detach().to(self.device, torch.float32)
-            if nm == "q" or not is_cross:
-                d["w" + nm] = P.pack_rows(w * gam[None, :], kept_c, C)
-                d["b" + nm] = self._pack_vec(w @ bet, kept_c, C)
-            else:
-                d["w" + nm] = P.pack_rows(w, kept_c, C)
+
+        def build(s, kept):
+            at, ls = self._src_mod(attn, s), self._src_mod(ln, s)
+            gam = ls.weight.detach().to(self.device, torch.float32)
+            bet = ls.bias.detach().to(self.device, torch.float32)
+            if not self.ln_fold:
+                gam, bet = torch.ones_like(gam), torch.zeros_like(bet)
+            o = {}
+            for nm, lin in (("q", at.to_q), ("k", at.to_k), ("v", at.to_v)):
+                w = lin.weight.detach().to(self.device, torch.float32)
+                if nm == "q" or not is_cross:
+                    o["w" + nm] = P.pack_rows(w * gam[None, :], kept, C)
+                    o["b" + nm] = self._pack_vec(w @ bet, kept, C)
+                else:
+                    o["w" + nm] = P.pack_rows(w, kept, C)
+            o["wo"] = P.pack_cols(at.to_out[0].weight.detach().to(self.device, BF16), kept, 1)
+            return o
+        d.update(self._variant_packs(vid, kept_c, build))
         if is_cross:
             d["cq"] = d["wq"].float().sum(1).contiguous()
             d["wkv"] = torch.cat([d["wk"], d["wv"]], 0).contiguous()
@@ -1491,8 +1583,7 @@ class _Engine:
             d["wqkv"] = torch.cat([d["wq"], d["wk"], d["wv"]], 0).contiguous()
             d["bqkv"] = torch.cat([d["bq"], d["bk"], d["bv"]], 0).contiguous()
             d["cqkv"] = d["wqkv"].float().sum(1).contiguous()
-        d["wo"] = P.pack_cols(attn.to_out[0].weight.detach().to(self.device, BF16), kept_c, 1)
-        d["bo"] = attn.to_out[0].bias.detach().to(self.device, torch.float32).contiguous()
+        d["bo"] = self._src_stack(attn, lambda at: at.to_out[0].bias.detach().to(self.device, torch.float32).contiguous())
         self.expert[key] = d
         return d
 
@@ -1508,7 +1599,7 @@ class _Engine:
         gw = ff.net[0].gate.width
         gs = inner // gw
         if self.compact:
-            kept_g, vid = P.kept_variants(self.eset.width_bits(gate_idx))
+            kept_g, vid = P.kept_variants(self.eset.width_bits(gate_idx), self.eset.source)
         else:
             kept_g, vid = [np.arange(gw)], np.zeros(1, dtype=np.int64)
         kept_c = [P.expand_groups(k, gs) for k in kept_g]
@@ -1516,7 +1607,20 @@ class _Engine:
         bn = P.choose_bn(list(nf), geglu=True, k=C)
         half = bn // 2
         rows_pad = ((inner + half - 1) // half) * bn
+        d = {"vid": vid, "nf": nf, "V": len(kept_c), "bn": bn, "rows_pad": rows_pad, "inner": inner, "gs": gs}
+        d.update(self._variant_packs(vid, kept_c, lambda s, kept: self._ff_blocks(
+            self._src_mod(ff, s), self._src_mod(ln, s), kept, C, inner, bn, rows_pad)))
+        d["sp"] = d["wp"].float().sum(1).contiguous()
+        d["b2"] = self._src_stack(ff, lambda f: f.net[2].bias.detach().to(self.device, torch.float32).contiguous())
+        self.expert[key] = d
+        return d
+
+    def _ff_blocks(self, ff: _FeedForward, ln: nn.LayerNorm, kept_c: List[np.ndarray], C: int, inner: int, bn: int,
+                   rows_pad: int) -> Dict[str, torch.Tensor]:
+        """GEGLU proj (norm3 folded in) and net.2 blocks of the variants `kept_c`, from the weights of `ff` / `ln`."""
+        half = bn // 2
         V = len(kept_c)
+        proj = ff.net[0].proj
         w = proj.weight.detach().to(self.device, torch.float32)
         gam = ln.weight.detach().to(self.device, torch.float32)
         bet = ln.bias.detach().to(self.device, torch.float32)
@@ -1543,15 +1647,13 @@ class _Engine:
             bblk = torch.stack([hb.view(nt, half), gb.view(nt, half)], dim=1).reshape(nt * bn)
             wp[v * rows_pad: v * rows_pad + nt * bn] = blk
             bp[v * rows_pad: v * rows_pad + nt * bn] = bblk
-        d = {"vid": vid, "nf": nf, "V": V, "bn": bn, "rows_pad": rows_pad, "wp": wp, "bp": bp, "inner": inner,
-             "gs": gs, "sp": wp.float().sum(1).contiguous()}
-        d["w2"] = P.pack_cols(ff.net[2].weight.detach().to(self.device, BF16), kept_c, 1)
-        d["b2"] = ff.net[2].bias.detach().to(self.device, torch.float32).contiguous()
-        self.expert[key] = d
-        return d
+        return {"wp": wp, "bp": bp, "w2": P.pack_cols(ff.net[2].weight.detach().to(self.device, BF16), kept_c, 1)}
 
     def _layernorm(self, tok: torch.Tensor, ln: nn.LayerNorm, M: int, C: int, hw: int, active: np.ndarray) -> torch.Tensor:
         """Un-folded LayerNorm pass (APTP_LN_FOLD=0 only): tok -> normalised bf16 rows."""
+        if len(self.srcs) > 1:
+            raise NotImplementedError("APTP_LN_FOLD=0 has one LayerNorm affine per launch: it cannot serve several "
+                                      "weight sources in one batch")
         key = ("ln_affine", id(ln))
         d = self.dense.get(key)
         if d is None:
@@ -1614,7 +1716,8 @@ class _Engine:
                     segs += self._segments(hw, nv, [(kq + 63) // 64] * E, off, vec_off=off, active=active,
                                            out_col_off=j * C)
                 s["qkv"] = K.build_schedule(segs, bn, self.device)
-            s["o"] = K.build_schedule(self._segments(hw, [C] * E, [int(n) for n in nh_e], vid * C, active=active),
+            s["o"] = K.build_schedule(self._segments(hw, [C] * E, [int(n) for n in nh_e], vid * C,
+                                                     vec_off=self._src_off(C), active=active),
                                       P.choose_bn([C], k=64 * int(max(pk["nh"]))), self.device)
             heads = np.where(active, nh_e, 0) if self.compact else np.asarray([attn.heads])
             s["heads"] = self._per_pos(heads) if self.compact else torch.full((B,), attn.heads, device=self.device,
@@ -1672,7 +1775,8 @@ class _Engine:
         dn = self.dense.get(key)
         if dn is None:
             f32 = lambda p: p.detach().to(self.device, torch.float32).contiguous()
-            dn = {"g": f32(t.norm.weight), "b": f32(t.norm.bias)}
+            dn = {"g": self._src_stack(t, lambda ts: f32(ts.norm.weight)),
+                  "b": self._src_stack(t, lambda ts: f32(ts.norm.bias))}
             for i, ln in enumerate((tb.norm1, tb.norm2, tb.norm3)):
                 dn[f"lg{i}"], dn[f"lb{i}"] = f32(ln.weight), f32(ln.bias)
             self.dense[key] = dn
@@ -1689,7 +1793,7 @@ class _Engine:
         xn = self.buf("ln", M, C)
         n_act = float(active[self.layout.expert_of_pos].sum()) if self.compact else float(B)
         self.groupnorm(x.f, C, C, B, hw, t.groups, gs, 1e-6, dn["g"], dn["b"], C, xn, C, False,
-                       sample_channels=aux["ch"], alg_elems=n_act * hw * C, cs0=x.cs)
+                       sample_seg=self._src_seg(), sample_channels=aux["ch"], alg_elems=n_act * hw * C, cs0=x.cs)
         tok = self.buf("tok", M, C)
         # LayerNorm statistics travel with the token stream: every GEMM that writes `tok` also writes per-row
         # (sum, sumsq) partials per 32-column chunk, and the three LayerNorms of the block (norm1/2/3, blocks.py:782,
@@ -1713,7 +1817,8 @@ class _Engine:
                                n_store=[min(P.round_up(int(n), 64), inner) for n in nf_e], active=active),
                 fk["bn"], self.device, geglu=True)
             s["o"] = K.build_schedule(
-                self._segments(hw, [C] * E, [(int(n) + 63) // 64 for n in nf_e], vid * C, active=active),
+                self._segments(hw, [C] * E, [(int(n) + 63) // 64 for n in nf_e], vid * C, vec_off=self._src_off(C),
+                               active=active),
                 P.choose_bn([C], k=int(max(fk["nf"]))), self.device)
             return s
         s = self._sched(("ff", t.uid, hw), build_ff)
@@ -1846,14 +1951,17 @@ class _Engine:
         self.launches += 1
         d = self.dense.get("conv_in")
         if d is None:
-            w = m.conv_in.weight.detach().to(self.device)
-            wp = torch.zeros(c0, 64, device=self.device, dtype=BF16)
-            wp[:, :9 * cin] = w.permute(0, 2, 3, 1).reshape(c0, 9 * cin).to(BF16)
-            d = {"w": wp, "b": m.conv_in.bias.detach().to(self.device, torch.float32).contiguous()}
+            def conv_in_w(conv):
+                wp = torch.zeros(c0, 64, device=self.device, dtype=BF16)
+                wp[:, :9 * cin] = conv.weight.detach().to(self.device).permute(0, 2, 3, 1).reshape(c0, 9 * cin).to(BF16)
+                return wp
+            d = {"w": self._src_stack(m.conv_in, conv_in_w),
+                 "b": self._src_stack(m.conv_in, lambda c: c.bias.detach().to(self.device, torch.float32).contiguous())}
             self.dense["conv_in"] = d
         x0 = torch.empty(B * H * W, c0, device=self.device, dtype=torch.float32)
+        E = self.eset.n_experts if self.compact else 1
         sched = self._sched(("conv_in", H, W), lambda: K.build_schedule(
-            [K.Segment(0, B * H * W, c0, 1)], P.choose_bn([c0]), self.device))
+            self._segments(H * W, [c0] * E, [1] * E, **self._dense_offs(m.conv_in)), P.choose_bn([c0]), self.device))
         cs0 = self._colstat_new(B, H, W, c0)
         self._gemm(sched, col, d["w"], x0, a_ld=64, a_k=64, a_rows=B * H * W, out_ld=c0, out_mode=OUT_F32, bias=d["b"],
                    rows_per_sample=H * W, colstat=cs0)
@@ -1873,18 +1981,20 @@ class _Engine:
         key = "out_norm"
         dn = self.dense.get(key)
         if dn is None:
-            dn = {"g": m.conv_norm_out.weight.detach().to(self.device, torch.float32).contiguous(),
-                  "b": m.conv_norm_out.bias.detach().to(self.device, torch.float32).contiguous()}
+            dn = {"g": self._src_stack(m.conv_norm_out, lambda n: n.weight.detach().to(self.device, torch.float32)),
+                  "b": self._src_stack(m.conv_norm_out, lambda n: n.bias.detach().to(self.device, torch.float32))}
+            dn = {k: v.contiguous() for k, v in dn.items()}
             self.dense[key] = dn
         groups = m.config["norm_num_groups"]
         a = self.buf("gn_a", x.rows, x.C)
         self.groupnorm(x.f, x.C, x.C, B, x.hw, groups, x.C // groups, m.config["norm_eps"], dn["g"], dn["b"], x.C, a,
-                       x.C, True, cs0=x.cs)
+                       x.C, True, sample_seg=self._src_seg(), cs0=x.cs)
         cout = m.config["out_channels"]
         y = torch.empty(B, cout, x.H, x.W, device=self.device, dtype=torch.float32)
         dco = self._dense_linear("conv_out", m.conv_out, n_pad_to=32)
         sched = self._sched(("conv_out", x.H, x.W), lambda: K.build_schedule(
-            [K.Segment(0, x.rows, cout, (x.C + 63) // 64)], 32, self.device, mode=A_CONV3X3, Ho=x.H, Wo=x.W))
+            self._segments(x.hw, [cout] * E, [(x.C + 63) // 64] * E, **self._dense_offs(m.conv_out, 32)), 32,
+            self.device, mode=A_CONV3X3, Ho=x.H, Wo=x.W))
         self._gemm(sched, a, dco["w"], y, a_ld=x.C, a_k=x.C, a_rows=x.rows, mode=A_CONV3X3, batch=B, H=x.H, W=x.W,
                    k_tap_pitch=x.C, out_ld=cout, out_mode=OUT_F32_NCHW, bias=dco["b"], rows_per_sample=x.hw)
         taps = []

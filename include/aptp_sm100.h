@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define APTP_ABI_VERSION 1
+#define APTP_ABI_VERSION 2
 
 /* library / diagnostics */
 int aptp_version(void);
@@ -54,7 +54,8 @@ typedef struct aptp_gemm_seg {
   int32_t vec_off;   /* offset of this bucket's bias (floats) in `bias`                           */
   int32_t tab_off;   /* offset of this bucket's 9 x n border table (floats) in `border_tab`       */
   int32_t out_col_off; /* output / residual column of this bucket's column 0 (fused q|k|v blocks)   */
-  int32_t pad0, pad1, pad2;
+  int32_t w2_row_off;  /* first row of this bucket's block in `w2` (second operand pair, a2 / w2)     */
+  int32_t pad1, pad2;
 } aptp_gemm_seg;
 
 typedef struct aptp_gemm_tile {
