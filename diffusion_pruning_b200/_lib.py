@@ -46,6 +46,10 @@ class GemmArgs(C.Structure):
     ]
 
 
+class SamplerCoeffs(C.Structure):
+    _fields_ = [(n, c_float) for n in ("sa", "sb", "c_x", "c_0", "c_h", "c_e", "c_n")]
+
+
 A_LINEAR, A_CONV3X3, A_CONV3X3_S2 = 0, 1, 2
 OUT_BF16, OUT_F32, OUT_F32_NCHW = 0, 1, 2
 EPI_GEGLU, EPI_SILU, EPI_GN_STATS, EPI_RES_F32, EPI_LN_FOLD = 1, 2, 4, 8, 16
@@ -86,6 +90,9 @@ SIGNATURES = {
     "aptp_cast_f32_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "aptp_silu_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "aptp_cfg_ddim_step": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_float, c_float, c_float, c_int, c_void_p]),
+    "aptp_cfg_pred_stats": (c_int, [c_void_p, c_int64, c_int, c_float, c_void_p, c_void_p]),
+    "aptp_cfg_sampler_step": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_float, c_float, c_void_p,
+                                      C.POINTER(SamplerCoeffs), c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p]),
     "aptp_attention_fwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
                                    c_int, c_void_p, c_int, c_float, c_void_p, c_void_p]),
     "aptp_attention_bwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int,

@@ -423,6 +423,24 @@ def cfg_ddim_step(pred, x, x_out, n, guidance, alpha_t, alpha_prev, v_prediction
                                     float(alpha_prev), int(v_prediction), _stream()), "aptp_cfg_ddim_step")
 
 
+SAMPLER_STAT_CHUNKS = 16  # APTP_SAMPLER_STAT_CHUNKS
+
+
+def cfg_pred_stats(pred, n_per_sample, batch, guidance, partials):
+    """partials [batch, SAMPLER_STAT_CHUNKS, 4] fp64: chunk sums of m_text, m_text^2, m, m^2 (guidance rescale)."""
+    check(load().aptp_cfg_pred_stats(_ptr(pred), n_per_sample, batch, float(guidance), _ptr(partials), _stream()),
+          "aptp_cfg_pred_stats")
+
+
+def cfg_sampler_step(pred, x, x_out, n_per_sample, batch, guidance, rescale, partials, coeffs, x0_hist_in=None,
+                     x0_hist_out=None, noise=None, noise_ld=0, v_prediction=True):
+    """One CFG (+ rescale) scheduler step; coeffs = (sa, sb, c_x, c_0, c_h, c_e, c_n) of sampling.sampler_plan."""
+    c = _lib.SamplerCoeffs(*[float(v) for v in coeffs])
+    check(load().aptp_cfg_sampler_step(_ptr(pred), _ptr(x), _ptr(x_out), n_per_sample, batch, float(guidance),
+                                       float(rescale), _ptr(partials), C.byref(c), _ptr(x0_hist_in), _ptr(x0_hist_out),
+                                       _ptr(noise), noise_ld, int(v_prediction), _stream()), "aptp_cfg_sampler_step")
+
+
 def attention(q, ldq, k, ldk, v, ldv, out, ldo, batch, n_q, n_kv, sample_heads, max_heads, scale, lse2=None):
     check(load().aptp_attention_fwd(_ptr(q), ldq, _ptr(k), ldk, _ptr(v), ldv, _ptr(out), ldo, batch, n_q, n_kv,
                                     _ptr(sample_heads), max_heads, float(scale), _ptr(lse2), _stream()),

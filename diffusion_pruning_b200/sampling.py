@@ -14,7 +14,8 @@ cluster_scripts/slurm/img_generation/sd2-1_cc3m.slurm:45-60).
 """
 from __future__ import annotations
 
-from typing import List, Optional, Tuple
+import math
+from typing import List, NamedTuple, Optional, Tuple
 
 import torch
 import torch.distributed as dist
@@ -27,6 +28,85 @@ def ddim_timesteps(num_inference_steps: int, num_train_timesteps: int = 1000, st
     """DDIMScheduler.set_timesteps with the SD-2.1 scheduler config ("leading" spacing, steps_offset 1)."""
     ratio = num_train_timesteps // num_inference_steps
     return [int(i * ratio) + steps_offset for i in range(num_inference_steps)][::-1]
+
+
+SCHEDULERS = ("ddim", "dpmsolver++")
+
+
+class SamplerStep(NamedTuple):
+    """One step of a sampling loop: the model runs at timestep t; coeffs = (sa, sb, c_x, c_0, c_h, c_e, c_n) are the
+    arguments of kernels.cfg_sampler_step; store_x0: the step keeps its x0 for the next (second-order) step."""
+    t: int
+    coeffs: Tuple[float, float, float, float, float, float, float]
+    store_x0: bool
+
+
+def sampler_plan(scheduler: str, steps: int, eta: float = 0.0, solver_order: int = 2,
+                 acp: Optional[torch.Tensor] = None) -> List[SamplerStep]:
+    """Per-step coefficients of x_prev = c_x x + c_0 x0 + c_h x0_last + c_e eps + c_n z on the ddim_timesteps(steps) grid
+    (the last step goes to acp[0]), computed once in float64. With abar = alphas_cumprod, a = sqrt(abar),
+    s = sqrt(1 - abar), lambda = log(a / s), t the current and p the previous timestep:
+      "ddim" (DDIMScheduler.step):  std = eta sqrt((1 - abar_p) / (1 - abar_t) (1 - abar_t / abar_p)),
+                                    x_prev = a_p x0 + sqrt(1 - abar_p - std^2) eps + std z
+      "dpmsolver++" (multistep, data prediction, midpoint form): h = lambda_p - lambda_t,
+                                    x_prev = (s_p / s_t) x - a_p (e^-h - 1) D,
+        D = x0 at order 1, D = (1 + 1/2r) x0 - (1/2r) x0_last with r = h_last / h at order 2. The first step is order
+        1, and so is the last when steps < 15 (lower_order_final).
+    x0 and eps are derived from the guided model output as in cfg_ddim_step (sa = a_t, sb = s_t)."""
+    _check_sampler_args(scheduler, eta, 0.0, solver_order)
+    acp = (alphas_cumprod() if acp is None else acp).detach().double().cpu()
+    ratio = 1000 // steps
+    plan, h_last = [], None
+    for i, t in enumerate(ddim_timesteps(steps)):
+        ab_t = float(acp[t])
+        ab_p = float(acp[t - ratio]) if t - ratio >= 0 else float(acp[0])   # set_alpha_to_one = False
+        sa, sb, ap, sp = math.sqrt(ab_t), math.sqrt(1.0 - ab_t), math.sqrt(ab_p), math.sqrt(1.0 - ab_p)
+        if scheduler == "ddim":
+            std = eta * math.sqrt((1.0 - ab_p) / (1.0 - ab_t) * (1.0 - ab_t / ab_p))
+            plan.append(SamplerStep(t, (sa, sb, 0.0, ap, 0.0, math.sqrt(1.0 - ab_p - std * std), std), False))
+            continue
+        h = math.log(ap / sp) - math.log(sa / sb)
+        phi = -ap * math.expm1(-h)
+        second = solver_order == 2 and i > 0 and not (i == steps - 1 and steps < 15)
+        if second:
+            r = h_last / h
+            c_0, c_h = phi * (1.0 + 0.5 / r), -phi * 0.5 / r
+        else:
+            c_0, c_h = phi, 0.0
+        plan.append(SamplerStep(t, (sa, sb, sp / sb, c_0, c_h, 0.0, 0.0), solver_order == 2 and i < steps - 1))
+        h_last = h
+    return plan
+
+
+def draw_step_noise(generator, steps: int, B: int, shape, device) -> torch.Tensor:
+    """The noise every step of a stochastic scheduler draws, drawn up front: [B, steps, *shape] fp32 on `device`.
+    Same order as diffusers' randn_tensor(model_output.shape, generator) once per step: step-major; with a list of
+    generators prompt b's rows come from generator[b] (drawn on that generator's device), with one generator (or None:
+    the global RNG, on `device`) each step is one batch draw. Every prompt thus sees the sequence the diffusers pipeline
+    would give it. Memory: steps x B x 4 x prod(shape) bytes (59 MB at 16 prompts, 4x96x96 latents, 25 steps)."""
+    shape = tuple(shape)
+    out = torch.empty(B, steps, *shape, device=device, dtype=torch.float32)
+    for i in range(steps):
+        if isinstance(generator, (list, tuple)):
+            for b, g in enumerate(generator):
+                out[b, i] = torch.randn((1, *shape), generator=g, device=g.device)[0].to(device)
+        else:
+            dev = device if generator is None else generator.device
+            out[:, i] = torch.randn((B, *shape), generator=generator, device=dev).to(device)
+    return out
+
+
+def _check_sampler_args(scheduler, eta, guidance_rescale, solver_order, generator=None, B=None) -> None:
+    if scheduler not in SCHEDULERS:
+        raise ValueError(f"scheduler must be one of {SCHEDULERS}, got {scheduler!r}")
+    if eta < 0 or (eta > 0 and scheduler != "ddim"):
+        raise ValueError(f"eta must be >= 0 and is a DDIM option (scheduler={scheduler!r}, eta={eta})")
+    if not 0.0 <= guidance_rescale <= 1.0:
+        raise ValueError(f"guidance_rescale must lie in [0, 1], got {guidance_rescale}")
+    if solver_order not in (1, 2):
+        raise ValueError(f"solver_order must be 1 or 2, got {solver_order}")
+    if isinstance(generator, (list, tuple)) and len(generator) != B:
+        raise ValueError(f"got {len(generator)} generators for {B} prompts")
 
 
 @torch.no_grad()
@@ -42,12 +122,24 @@ def route_prompts(hyper_net, quantizer, prompt_embeddings: torch.Tensor) -> Tupl
 def denoise(unet, hyper_net, arch_vectors: torch.Tensor, latents: torch.Tensor, cond: torch.Tensor,
             uncond: torch.Tensor, num_inference_steps: int = 25, guidance_scale: float = 7.5,
             acp: Optional[torch.Tensor] = None, prediction_type: str = "v_prediction", experts=None,
-            expert_index: Optional[torch.Tensor] = None) -> torch.Tensor:
+            expert_index: Optional[torch.Tensor] = None, *, scheduler: str = "ddim", eta: float = 0.0,
+            generator=None, guidance_rescale: float = 0.0, solver_order: int = 2,
+            step_noise: Optional[torch.Tensor] = None) -> torch.Tensor:
     """The scheduler loop (pruning_pipelines.py:757-820) for one batch of prompts whose hard architecture
     vectors are `arch_vectors` (any mix of experts). latents [B,4,H,W] fp32 ~ N(0,1) (init_noise_sigma = 1).
     With `experts` (a PrunedExpertMixture) each prompt runs on its fine-tuned expert `expert_index` [B] instead: `unet`,
-    `hyper_net` and `arch_vectors` are not used."""
+    `hyper_net` and `arch_vectors` are not used.
+
+    The pipeline's scheduler controls (sampler_plan has the definitions):
+      scheduler: "ddim" or "dpmsolver++" (DPMSolverMultistepScheduler, data prediction; solver_order 1 or 2);
+      eta: DDIM noise level (>= 0); the noise of every step comes from `generator` (None, one torch.Generator or a list
+           of B, one per prompt) in draw_step_noise's order, or is given as step_noise [B, steps, 4, H, W] fp32
+           (steps x B x 16 H W bytes: 59 MB at 16 prompts, 96x96 latents, 25 steps);
+      guidance_rescale: diffusers rescale_noise_cfg factor in [0, 1].
+    The defaults (DDIM, eta 0, no rescale) run the fused cfg_ddim_step loop; anything else runs cfg_sampler_step (and
+    cfg_pred_stats when guidance_rescale > 0)."""
     B = latents.shape[0]
+    _check_sampler_args(scheduler, eta, guidance_rescale, solver_order, generator, B)
     if B == 0:
         return latents
     acp = (alphas_cumprod() if acp is None else acp).cpu()
@@ -64,6 +156,9 @@ def denoise(unet, hyper_net, arch_vectors: torch.Tensor, latents: torch.Tensor, 
     x = latents.float().contiguous()
     x2 = torch.empty(2 * B, *x.shape[1:], device=x.device, dtype=torch.float32)
     nxt = torch.empty_like(x)
+    if scheduler != "ddim" or eta != 0 or guidance_rescale != 0:
+        return _sampler_loop(model, emb, x, x2, nxt, num_inference_steps, guidance_scale, acp, prediction_type,
+                             scheduler, eta, generator, guidance_rescale, solver_order, step_noise)
     for t in ts:                                                             # :790
         x2[:B].copy_(x)                                                      # :792 cat([latents] * 2)
         x2[B:].copy_(x)
@@ -74,6 +169,37 @@ def denoise(unet, hyper_net, arch_vectors: torch.Tensor, latents: torch.Tensor, 
         a_prev = float(acp[prev]) if prev >= 0 else float(acp[0])            # set_alpha_to_one = False
         K.cfg_ddim_step(pred.contiguous(), x, nxt, x.numel(), guidance_scale, a_t, a_prev,
                         prediction_type == "v_prediction")                   # :805-814 fused
+        x, nxt = nxt, x
+    return x
+
+
+def _sampler_loop(model, emb, x, x2, nxt, steps, guidance_scale, acp, prediction_type, scheduler, eta, generator,
+                  guidance_rescale, solver_order, step_noise):
+    B, n = x.shape[0], x[0].numel()
+    x = x.clone()   # the ping-pong writes into x every other step; it may be the caller's latents
+    plan = sampler_plan(scheduler, steps, eta, solver_order, acp)
+    noise = None
+    if eta > 0:
+        if step_noise is None:
+            step_noise = draw_step_noise(generator, steps, B, x.shape[1:], x.device)
+        if tuple(step_noise.shape) != (B, steps, *x.shape[1:]):
+            raise ValueError(f"step_noise must be [{B}, {steps}, {', '.join(map(str, x.shape[1:]))}], "
+                             f"got {list(step_noise.shape)}")
+        noise = step_noise.to(x.device, torch.float32).contiguous()
+    hist = torch.empty_like(x) if any(st.store_x0 for st in plan) else None
+    partials = (torch.empty(B, K.SAMPLER_STAT_CHUNKS, 4, device=x.device, dtype=torch.float64)
+                if guidance_rescale > 0 else None)
+    vpred = prediction_type == "v_prediction"
+    for i, st in enumerate(plan):
+        x2[:B].copy_(x)
+        x2[B:].copy_(x)
+        tt = torch.full((2 * B,), float(st.t), device=x.device)
+        pred = model(x2, tt, emb).sample.contiguous()
+        if partials is not None:
+            K.cfg_pred_stats(pred, n, B, guidance_scale, partials)
+        K.cfg_sampler_step(pred, x, nxt, n, B, guidance_scale, guidance_rescale, partials, st.coeffs,
+                           hist if st.coeffs[4] != 0 else None, hist if st.store_x0 else None,
+                           None if noise is None else noise[:, i], 0 if noise is None else noise.stride(0), vpred)
         x, nxt = nxt, x
     return x
 
@@ -121,13 +247,25 @@ def _all_to_all_rows(t: torch.Tensor, send_counts: List[int], recv_counts: List[
 def routed_sampling(unet, hyper_net, quantizer, prompt_embeddings: torch.Tensor, latents: torch.Tensor,
                     cond: torch.Tensor, uncond: torch.Tensor, num_inference_steps: int = 25,
                     guidance_scale: float = 7.5, acp: Optional[torch.Tensor] = None, dispatch: str = "balanced",
-                    experts=None, code_to_expert: Optional[torch.Tensor] = None):
+                    experts=None, code_to_expert: Optional[torch.Tensor] = None, *, scheduler: str = "ddim",
+                    eta: float = 0.0, generator=None, guidance_rescale: float = 0.0, solver_order: int = 2):
     """BASELINE configs[3]: route local prompts, dispatch them (all-to-all over NVLink) to the GPU chosen by
     plan_dispatch -- the rank(s) serving their expert, load-balanced --, denoise there, return the final latents to
     the rank that asked. Returns (latents, code index).
     With `experts` (a PrunedExpertMixture, held whole by every rank) each prompt is denoised by the fine-tuned expert of
     its routed code: `code_to_expert` [n_codes] maps a code index to a mixture position (default:
-    experts.code_to_expert(quantizer.n_e), from the experts' code ids). Routing and dispatch are unchanged."""
+    experts.code_to_expert(quantizer.n_e), from the experts' code ids). Routing and dispatch are unchanged.
+    scheduler / eta / generator / guidance_rescale / solver_order are denoise's. With eta > 0 the asking rank draws
+    every step's noise of its prompts up front (draw_step_noise: one generator for the batch or one per prompt) and
+    ships it with the prompts, so a prompt gets the same noise whichever rank serves it."""
+    B = latents.shape[0]
+    _check_sampler_args(scheduler, eta, guidance_rescale, solver_order, generator, B)
+    sampler_kw = {k: v for k, v, default in (("scheduler", scheduler, "ddim"), ("eta", eta, 0.0),
+                                             ("guidance_rescale", guidance_rescale, 0.0),
+                                             ("solver_order", solver_order, 2)) if v != default}
+    step_noise = None
+    if eta > 0:
+        step_noise = draw_step_noise(generator, num_inference_steps, B, latents.shape[1:], latents.device)
     arch, idx = route_prompts(hyper_net, quantizer, prompt_embeddings)
     eidx = None
     if experts is not None:
@@ -139,7 +277,10 @@ def routed_sampling(unet, hyper_net, quantizer, prompt_embeddings: torch.Tensor,
     world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     if world == 1:
         kw = {} if experts is None else dict(experts=experts, expert_index=eidx)
-        return denoise(unet, hyper_net, arch, latents, cond, uncond, num_inference_steps, guidance_scale, acp, **kw), idx
+        if step_noise is not None:
+            kw["step_noise"] = step_noise
+        return denoise(unet, hyper_net, arch, latents, cond, uncond, num_inference_steps, guidance_scale, acp, **kw,
+                       **sampler_kw), idx
     owner = plan_dispatch(idx, quantizer.n_e, dispatch)
     order = torch.argsort(owner, stable=True)
     send = torch.bincount(owner, minlength=world)
@@ -147,11 +288,13 @@ def routed_sampling(unet, hyper_net, quantizer, prompt_embeddings: torch.Tensor,
     dist.all_to_all_single(recv, send)
     sc, rc = send.tolist(), recv.tolist()
     payload = [arch[order], latents[order].float(), cond[order], uncond[order]]
-    if eidx is not None:
-        payload.append(eidx[order])
-    arch_r, lat_r, cond_r, unc_r, *eidx_r = [_all_to_all_rows(p, sc, rc) for p in payload]
-    kw = {} if experts is None else dict(experts=experts, expert_index=eidx_r[0])
-    out_r = denoise(unet, hyper_net, arch_r, lat_r, cond_r, unc_r, num_inference_steps, guidance_scale, acp, **kw)
+    extra = [(k, t) for k, t in (("expert_index", eidx), ("step_noise", step_noise)) if t is not None]
+    arch_r, lat_r, cond_r, unc_r, *extra_r = [_all_to_all_rows(p, sc, rc) for p in payload + [t[order] for _, t in extra]]
+    kw = dict(zip([k for k, _ in extra], extra_r))
+    if experts is not None:
+        kw["experts"] = experts
+    out_r = denoise(unet, hyper_net, arch_r, lat_r, cond_r, unc_r, num_inference_steps, guidance_scale, acp, **kw,
+                    **sampler_kw)
     back = _all_to_all_rows(out_r, rc, sc)
     out = torch.empty_like(back)
     out[order] = back

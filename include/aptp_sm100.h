@@ -261,6 +261,30 @@ int aptp_silu_bf16(const void* src, void* dst, int64_t n, void* stream);
  * alphas_cumprod at the current / previous timestep. */
 int aptp_cfg_ddim_step(const float* pred, const float* x, float* x_out, int64_t n, float guidance, float alpha_t,
                        float alpha_prev, int32_t v_prediction, void* stream);
+/* Scheduler steps beyond DDIM eta 0 (csrc/sampler.cu): stochastic DDIM, DPM-Solver++ (1 / 2M) and guidance rescale
+ * (diffusers DDIMScheduler.step, DPMSolverMultistepScheduler, rescale_noise_cfg). `pred` is the [uncond B | cond B]
+ * fp32 NCHW block; every sample has n_per_sample (a multiple of 4) elements; all pointers 16-byte aligned.
+ *
+ * aptp_cfg_pred_stats: partials[batch][APTP_SAMPLER_STAT_CHUNKS][4] (fp64) = per-chunk sums of m_text, m_text^2, m,
+ * m^2 with m_text = cond prediction and m = uncond + guidance (cond - uncond). Fixed summation order, no atomics: two
+ * runs on the same input are bit-identical.
+ *
+ * aptp_cfg_sampler_step: per element, m = uncond + guidance (cond - uncond); with `partials` (may be NULL) m is
+ * scaled by rescale * std(m_text) / std(m) + 1 - rescale, std the unbiased per-sample std from the partials; then
+ *   v-prediction:  x0 = sa x - sb m,   eps = sa m + sb x      epsilon: eps = m, x0 = (x - sb m) / sa
+ *   x_out = c_x x + c_0 x0 + c_h x0_hist_in + c_e eps + c_n noise,   x0_hist_out = x0 (when not NULL).
+ * x0_hist_in / noise may be NULL when c_h / c_n is 0; x0_hist_in may equal x0_hist_out; x_out must not alias x.
+ * noise holds sample b's elements at noise + b * noise_ld. `coeffs` is read at call time (host memory). */
+#define APTP_SAMPLER_STAT_CHUNKS 16
+typedef struct {
+  float sa, sb, c_x, c_0, c_h, c_e, c_n;
+} AptpSamplerCoeffs;
+int aptp_cfg_pred_stats(const float* pred, int64_t n_per_sample, int32_t batch, float guidance, double* partials,
+                        void* stream);
+int aptp_cfg_sampler_step(const float* pred, const float* x, float* x_out, int64_t n_per_sample, int32_t batch,
+                          float guidance, float rescale, const double* partials, const AptpSamplerCoeffs* coeffs,
+                          const float* x0_hist_in, float* x0_hist_out, const float* noise, int64_t noise_ld,
+                          int32_t v_prediction, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K3  flash-style attention on tcgen05 with per-sample kept-head lists.
