@@ -93,6 +93,9 @@ SIGNATURES = {
     "aptp_cfg_pred_stats": (c_int, [c_void_p, c_int64, c_int, c_float, c_void_p, c_void_p]),
     "aptp_cfg_sampler_step": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_float, c_float, c_void_p,
                                       C.POINTER(SamplerCoeffs), c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p]),
+    "aptp_cfg_sampler_step_masked": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_float, c_float, c_void_p,
+                                             C.POINTER(SamplerCoeffs), c_void_p, c_void_p, c_void_p, c_int64, c_int,
+                                             c_void_p, c_void_p, c_int64, c_void_p, c_float, c_float, c_void_p]),
     "aptp_attention_fwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
                                    c_int, c_void_p, c_int, c_float, c_void_p, c_void_p]),
     "aptp_attention_bwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int,

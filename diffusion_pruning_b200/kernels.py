@@ -441,6 +441,19 @@ def cfg_sampler_step(pred, x, x_out, n_per_sample, batch, guidance, rescale, par
                                        _ptr(noise), noise_ld, int(v_prediction), _stream()), "aptp_cfg_sampler_step")
 
 
+def cfg_sampler_step_masked(pred, x, x_out, n_per_sample, batch, guidance, rescale, partials, coeffs, image, mask,
+                            plane_size, init_noise, a_next, s_next, x0_hist_in=None, x0_hist_out=None, noise=None,
+                            noise_ld=0, v_prediction=True):
+    """cfg_sampler_step, then x_out = (1 - m) (a_next image + s_next init_noise) + m x_out in the same pass; mask is one
+    plane of plane_size floats per sample, broadcast over the channels (inpainting, 1 = regenerate)."""
+    c = _lib.SamplerCoeffs(*[float(v) for v in coeffs])
+    check(load().aptp_cfg_sampler_step_masked(_ptr(pred), _ptr(x), _ptr(x_out), n_per_sample, batch, float(guidance),
+                                              float(rescale), _ptr(partials), C.byref(c), _ptr(x0_hist_in),
+                                              _ptr(x0_hist_out), _ptr(noise), noise_ld, int(v_prediction), _ptr(image),
+                                              _ptr(mask), plane_size, _ptr(init_noise), float(a_next), float(s_next),
+                                              _stream()), "aptp_cfg_sampler_step_masked")
+
+
 def attention(q, ldq, k, ldk, v, ldv, out, ldo, batch, n_q, n_kv, sample_heads, max_heads, scale, lse2=None):
     check(load().aptp_attention_fwd(_ptr(q), ldq, _ptr(k), ldk, _ptr(v), ldv, _ptr(out), ldo, batch, n_q, n_kv,
                                     _ptr(sample_heads), max_heads, float(scale), _ptr(lse2), _stream()),

@@ -18,6 +18,8 @@ Execution model (B200-first, not a translation of the module-by-module eager ref
 """
 from __future__ import annotations
 
+import contextlib
+import gc
 import os
 
 import math
@@ -40,6 +42,21 @@ BF16 = torch.bfloat16
 @dataclass
 class UNet2DConditionOutput:
     sample: torch.Tensor
+
+
+@contextlib.contextmanager
+def _graph_capture(g):
+    """torch.cuda.graph(g) with Python's cyclic garbage collector held off for the capture. A collection inside the
+    capture can free an unreachable model whose engine holds captured graphs; destroying a graph is not permitted while
+    a (global-mode) capture is open, so it would invalidate this capture. The garbage is collected after the capture."""
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(g):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
 
 
 def _require_cuda(sample: torch.Tensor) -> None:
@@ -882,7 +899,7 @@ class _Engine:
         self._refresh_packs_eager()
         torch.cuda.synchronize()
         g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
+        with _graph_capture(g):
             self._refresh_packs_eager()
         self._pack_graph, self._pack_graph_n = g, len(self._packs)
         g.replay()
@@ -1900,7 +1917,7 @@ class _Engine:
             st_s, st_t, st_c = sample.clone(), timestep.clone(), ctx.clone()
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
+            with _graph_capture(g):
                 y, taps = self.run(st_s, st_t, st_c, want_taps)
             # the captured kernels read this state's schedules and packed weights: the graph keeps them alive even if
             # the LRU caches above drop the state in the meantime

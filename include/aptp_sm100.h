@@ -285,6 +285,20 @@ int aptp_cfg_sampler_step(const float* pred, const float* x, float* x_out, int64
                           float guidance, float rescale, const double* partials, const AptpSamplerCoeffs* coeffs,
                           const float* x0_hist_in, float* x0_hist_out, const float* noise, int64_t noise_ld,
                           int32_t v_prediction, void* stream);
+/* aptp_cfg_sampler_step_masked: aptp_cfg_sampler_step followed, in the same pass, by the inpainting blend
+ *   x_out = (1 - m) (a_next image + s_next init_noise) + m x_step
+ * with x_step the unmasked step's output and m = mask[b][j % plane_size] for element j of sample b (one plane of
+ * plane_size floats per sample, broadcast over the n_per_sample / plane_size channels; plane_size need not be a
+ * multiple of 4). m = 0 gives a_next image + s_next init_noise and m = 1 gives x_step bit for bit; a_next = 1,
+ * s_next = 0 gives image bit for bit where m = 0. x0_hist_out receives the x0 before the blend. image and init_noise
+ * are [batch][n_per_sample]; image, mask and init_noise are read only and must not alias x_out or x0_hist_out; the
+ * other aliasing rules are aptp_cfg_sampler_step's. */
+int aptp_cfg_sampler_step_masked(const float* pred, const float* x, float* x_out, int64_t n_per_sample, int32_t batch,
+                                 float guidance, float rescale, const double* partials,
+                                 const AptpSamplerCoeffs* coeffs, const float* x0_hist_in, float* x0_hist_out,
+                                 const float* noise, int64_t noise_ld, int32_t v_prediction, const float* image,
+                                 const float* mask, int64_t plane_size, const float* init_noise, float a_next,
+                                 float s_next, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K3  flash-style attention on tcgen05 with per-sample kept-head lists.
